@@ -47,7 +47,36 @@ def parse():
     p.add_argument("--lr", type=float, default=1e-4)
     p.add_argument("--train-gemm", default="tc", choices=["fp32", "bf16x3", "tc"],
                    help="training-path GEMMs: CUDA-core fp32 | split-bf16 mma.sync | split-bf16 with the edge-tensor GEMMs (forward, data and weight gradients) on tcgen05")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB in all) "
+                        "so that two builds can be compared output for output")
+    args = p.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.sweep):
+        p.error("--dump-outputs applies to the GPU sampling and training runs (not --impl reference or --sweep)")
+    return args
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def write_dump(path, arrays):
+    """Writes {name: float32 / float64 array} as path/<name>.npy."""
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT and all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+    print(f"[bench] wrote {', '.join(sorted(arrays))} to {path}", file=sys.stderr)
+
+
+def sample_subset(arrays):
+    """Arrays indexed by global sample on axis 0: all of them if they fit DUMP_LIMIT, else the same fixed seeded subset of samples of
+    each, whose indices go to sample_index."""
+    n = next(iter(arrays.values())).shape[0]
+    per_sample = sum(a.nbytes for a in arrays.values()) / n + 8
+    if per_sample * n <= DUMP_LIMIT:
+        return arrays
+    keep = np.sort(np.random.default_rng(0).choice(n, int(DUMP_LIMIT // per_sample), replace=False))
+    return dict({k: v[keep] for k, v in arrays.items()}, sample_index=keep.astype(np.float64))
 
 
 def peaks():
@@ -284,6 +313,13 @@ def run_train(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dev_s, e2e_s, exposed_ms = float(t[0]) / 1e3 / args.steps, float(t[1]) / 1e3 / args.steps, float(t[2]) / args.steps
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed step (the e2e leg of the last iteration): its loss, the parameters it updated in place and the gradients it
+        # computed (identical on every rank after the all-reduce); 17.4 M floats each, so a fixed seeded sample of 2 M positions
+        idx = np.sort(np.random.default_rng(0).choice(ts.params.numel(), 2_000_000, replace=False))
+        at = torch.from_numpy(idx).to(dev)
+        write_dump(args.dump_outputs, {"loss": np.array([losses[-1]], np.float64), "params": ts.params[at].cpu().numpy(),
+                                       "grads": ts.grads[at].cpu().numpy(), "param_index": idx.astype(np.float64)})
     if rank == 0:
         pk = peaks()
         fl = train_flops(B, N)
@@ -328,6 +364,7 @@ def sample_line(args, eng, state, B, N, T, prec, world, rank, local, dist, torch
         if world > 1:
             dist.all_gather_into_tensor(gathered, a37)
         last["a37"] = gathered if world > 1 else a37
+        last["rig"] = rig
         return ms, nl
 
     masks = {"res_mask": np.ones((B, N), np.float32), "fixed_mask": np.zeros((B, N), np.float32),
@@ -351,8 +388,11 @@ def sample_line(args, eng, state, B, N, T, prec, world, rank, local, dist, torch
         barrier(); dev_wall += time.perf_counter() - t0
         gpu_ms += ms; launches += nl
         barrier(); t0 = time.perf_counter()
-        e2e_step(2000 + i)
+        res = e2e_step(2000 + i)
         barrier(); e2e_wall += time.perf_counter() - t0
+        if i == steps - 1:          # earlier steps' pinned output buffers go back to the allocator before the next step, as without a dump
+            last["e2e"] = res
+        del res
     # the loop runs on the engine's own stream and is timed there with CUDA events (fd_sample_dev's gpu_ms); wall adds the host-side
     # launch overhead and, for N>1, the NCCL gather — report the larger (honest) one, max over ranks
     t = torch.tensor([max(dev_wall, gpu_ms / 1e3), e2e_wall], device=dev, dtype=torch.float64)
@@ -365,6 +405,18 @@ def sample_line(args, eng, state, B, N, T, prec, world, rank, local, dist, torch
     nchk = min(32, B)
     chk = last["a37"][:nchk].double().sum().item() if rank == 0 else None
     chk_abs = last["a37"][:nchk].double().abs().sum().item() if rank == 0 else None
+    if args.dump_outputs:
+        # the last timed step's results of both legs (device-resident loop; public API with host buffers), in global-sample order
+        e2e = last["e2e"]
+        out = {"atom37": last["a37"], "rigids": last["rig"], "e2e_atom37": torch.from_numpy(e2e["prot_traj"][0]).to(dev),
+               "e2e_rigids": torch.from_numpy(e2e["rigids_final"]).to(dev), "e2e_psi": torch.from_numpy(e2e["psi_pred"][0]).to(dev)}
+        if world > 1:          # after the timed region: the timed path gathers atom37 only
+            for k in ("rigids", "e2e_atom37", "e2e_rigids", "e2e_psi"):
+                g = out[k].new_empty((world * B,) + tuple(out[k].shape[1:]))
+                dist.all_gather_into_tensor(g, out[k].contiguous())
+                out[k] = g
+        if rank == 0:
+            write_dump(args.dump_outputs, sample_subset({k: v.cpu().numpy() for k, v in out.items()}))
     if rank != 0:
         return None
     roof = None

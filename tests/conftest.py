@@ -26,10 +26,8 @@ def golden(name):
 def paper_weights_path():
     """A copy of the reference's weights/paper_weights.pth as .npz, if one is available (it is an input artefact,
     70 MB, git-ignored; see tests/golden/export_paper_weights.py)."""
-    for p in (os.path.join(ROOT, "weights", "paper_weights.npz"), "/tmp/fd_weights/paper_weights.npz"):
-        if os.path.exists(p):
-            return p
-    return None
+    p = os.path.join(ROOT, "weights", "paper_weights.npz")
+    return p if os.path.exists(p) else None
 
 
 def assert_close(a, b, rtol, atol=0.0, name="", norm_rel=None):

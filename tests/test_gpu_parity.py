@@ -743,3 +743,40 @@ def test_sample_sharded_single_process_equals_sample_device(eng):
     first, count = shard_range(4, 2, 1)
     c37, _, _, _ = eng.sample_device(count, 40, num_t=5, seed=21, first_sample=first)
     assert_close(c37.cpu().numpy(), a37[first:first + count].cpu().numpy(), 0, norm_rel=1e-5, name="rank-1 shard of a 2-way split")
+
+
+@pytest.mark.parametrize("mode", ["sample", "train"])
+def test_bench_dump_outputs(tmp_path, mode):
+    """`bench.py --dump-outputs DIR` writes the last timed step's results as float .npy files; two runs with the same arguments use
+    the same inputs, so they agree (sampling: both legs of a step compute the same samples)."""
+    import json, os, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    extra = ["--num-t", "4", "--batch", "2"] if mode == "sample" else ["--batch", "1"]
+    runs = []
+    for k in range(2):
+        d = tmp_path / f"run{k}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1", "--mode", mode,
+                            "--nres", "40", "--no-cpu-baseline", "--dump-outputs", str(d)] + extra,
+                           cwd=tmp_path, capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
+        assert json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])["steps"] == 2
+        runs.append({f[:-4]: np.load(d / f) for f in sorted(os.listdir(d))})
+    a, b = runs
+    assert all(v.dtype in (np.float32, np.float64) and np.all(np.isfinite(v)) for v in a.values())
+    if mode == "sample":
+        assert sorted(a) == ["atom37", "e2e_atom37", "e2e_psi", "e2e_rigids", "rigids"]
+        assert a["atom37"].shape == (2, 40, 37, 3) and a["rigids"].shape == (2, 40, 7) and a["e2e_psi"].shape == (2, 40, 2)
+        assert_close(a["e2e_atom37"], a["atom37"], 0, norm_rel=1e-5, name="host-buffer leg vs device leg")
+        assert_close(a["e2e_rigids"][..., 4:], a["rigids"][..., 4:], 0, norm_rel=1e-5, name="host-buffer leg vs device leg")
+        for k in a:
+            assert_close(b[k], a[k], 0, norm_rel=1e-4, name=f"run 2 vs run 1: {k}")
+        return
+    assert sorted(a) == ["grads", "loss", "param_index", "params"]
+    assert a["params"].shape == a["grads"].shape == a["param_index"].shape == (2_000_000,) and np.all(np.diff(a["param_index"]) > 0)
+    assert np.array_equal(a["param_index"], b["param_index"])
+    # the backward's atomic sums differ in rounding from run to run, and Adam turns rounding noise in a near-zero gradient into a step
+    # of about lr: the runs agree to the tensor-core training mode's gradient accuracy, the parameters to 2 lr per Adam step
+    adam_steps = 1 + 2 * 2                      # the warm-up step, then both legs of each timed step
+    assert_close(b["params"], a["params"], 0, atol=2 * adam_steps * 1e-4, name="run 2 vs run 1: params")
+    assert_close(b["grads"], a["grads"], 0, norm_rel=6e-3, name="run 2 vs run 1: grads")
+    assert_close(b["loss"], a["loss"], 1e-3, name="run 2 vs run 1: loss")

@@ -95,6 +95,23 @@ print("OVERLAY-OK", len(net.state_dict()))
     assert "OVERLAY-OK 282" in out.stdout, out.stdout + out.stderr
 
 
+def test_state_dict_layout_equals_the_reference_module_and_shipped_checkpoints():
+    """Our module's state_dict has exactly the parameter names, order and shapes of the reference's ScoreNetwork and of both shipped
+    checkpoints (tests/golden/make_golden_overlay.py): the checkpoints load strict=True and the reference loads what our module writes."""
+    from conftest import golden
+    from se3_diffusion_b200.score_network import ScoreNetwork
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import ref_harness as rh
+    g = golden("state_dict_layout")
+    net = ScoreNetwork(rh.default_conf()[0], diffuser=None)
+    ours = [(k, tuple(v.shape)) for k, v in net.state_dict().items()]
+    for tag in ("module", "paper_weights", "best_weights"):
+        dims = iter(g[f"{tag}_dims"].tolist())
+        ref = [(str(n), tuple(next(dims) for _ in range(k))) for n, k in zip(g[f"{tag}_names"], g[f"{tag}_ndim"].tolist())]
+        assert ours == ref, tag
+        net.load_state_dict({n: torch.zeros(s) for n, s in ref}, strict=True)
+
+
 def test_shard_range_partitions_batch():
     from se3_diffusion_b200.parallel import shard_range
     for B in (1, 7, 32, 256):

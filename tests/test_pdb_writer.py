@@ -89,6 +89,22 @@ def test_overlay_module_next_to_reference(tmp_path):
         assert open(tmp_path / "r" / fn, "rb").read() == open(tmp_path / "o" / fn, "rb").read()
 
 
+def test_sampler_calls_write_the_reference_files(tmp_path):
+    """Called the way Sampler.save_traj calls the reference's writer (suffix-less paths, indexed names, b-factors 100 on diffused
+    residues), the native writer produces the files the unmodified reference wrote for the same trajectory
+    (tests/golden/make_golden_overlay.py)."""
+    g = golden("pdb_sampler_calls")
+    pos, bfac = g["pos"], g["b_factors"]
+    plain = pdb_writer.write_prot_to_pdb(pos, str(tmp_path / "ref.pdb"), no_indexing=True)
+    assert open(plain, "rb").read() == g["plain"].tobytes()
+    paths = [pdb_writer.write_prot_to_pdb(pos[0], str(tmp_path / "sample"), b_factors=bfac),
+             pdb_writer.write_prot_to_pdb(pos, str(tmp_path / "bb_traj"), b_factors=bfac),
+             pdb_writer.write_prot_to_pdb(pos[0], str(tmp_path / "sample"), b_factors=bfac)]
+    assert [os.path.basename(p) for p in paths] == [str(n) for n in g["names"]]
+    for p, key in zip(paths, ("sample", "traj", "sample")):
+        assert open(p, "rb").read() == g[key].tobytes(), os.path.basename(p)
+
+
 def test_fixed_point_formatter_equals_printf_on_hard_values():
     """fd_format_pdb's own %8.3f / %6.2f (scale, round-half-even, emit digits; snprintf near ties and beyond 9e15) against Python's
     correctly rounded formatting: float32-born values (exact ties possible), float64 values adjacent to decimal ties, zeros of both
